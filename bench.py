@@ -27,6 +27,9 @@ rank builds its partial moments, ONE all-reduce of the (p+2)^2 f64 moments over 
 the end-to-end leg too: each rank passes ITS host shard to the plugin symbol and the library fits ONE regression over
 N x rows.  C3 / C4 shard without a collective (groups / rows with a read-only halo).
 `--impl reference` times the CPU arm alone (rank 0 only), full-size steps.
+`--dump-outputs DIR` writes what the last timed step returned (coefficients, status, per-row outputs) as DIR/<name>.npy,
+at most 64 MB: per-row outputs longer than that keep a fixed seeded sample of rows.  Inputs are seeded, so two builds run
+with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -69,7 +72,13 @@ def parse_args():
     ap.add_argument("--cpu-steps", type=int, default=3, help="passes of the CPU baseline inside the ours arm")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rows, feats, dtype, desc = CONFIGS[a.config]
     a.rows = a.rows or rows
     a.features = a.features or feats
@@ -344,10 +353,10 @@ def cpu_other(args, steps, warmup, host=None):
             for _ in range(max(1, warmup)):
                 orc.pl_lr(cols, kw, f32=False)
             t0 = time.perf_counter()
-            for _ in range(max(steps, 20)):
+            for _ in range(steps):
                 orc.pl_lr(cols, kw, f32=False)
-            dt = (time.perf_counter() - t0) / max(steps, 20)
-        return n / dt, dt, (f"{max(steps, 20)} full-size passes of oracle.pl_lr (numpy/OpenBLAS, up to {host_threads()} BLAS "
+            dt = (time.perf_counter() - t0) / steps
+        return n / dt, dt, (f"{steps} full-size passes of oracle.pl_lr (numpy/OpenBLAS, up to {host_threads()} BLAS "
                             f"threads) on {n} x {p} f64 + bias, {dt * 1e3:.2f} ms each"), host_threads()
     if args.config == "C3":
         n_groups, gl = 200, 10_000
@@ -371,10 +380,9 @@ def cpu_other(args, steps, warmup, host=None):
     kw = {"null_policy": "raise", "n": 1024, "bias": False, "lambda": 0.0, "min_size": min(p, 1024)}
     with blas_threads(1):
         t0 = time.perf_counter()
-        reps = max(1, min(steps, 3))
-        for _ in range(reps):
+        for _ in range(steps):
             orc.pl_rolling_lr(cols, kw, f32=True)
-        dt = (time.perf_counter() - t0) / reps
+        dt = (time.perf_counter() - t0) / steps
     return n / dt, dt, (f"oracle.pl_rolling_lr (sequential Woodbury walk like faer_rolling_lr, ONE thread as in the reference) on "
                         f"a {n}-row slice x {p} f32, window 1024, {dt:.2f} s per pass; the walk is O(n), so rows/s carries to 1e8"), 1
 
@@ -460,6 +468,8 @@ def main():
     launches = dev.launch_count() - launches0
     ms = max_over_ranks(ev0.elapsed_time(ev1))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, w["outputs"]())
     rows = args.rows
     value = rows * world * args.steps / (ms * 1e-3)
 
@@ -575,6 +585,30 @@ def host_copy(torch, dev_rows, pinned):
     return out
 
 
+DUMP_BYTES = 60 << 20       # --dump-outputs stays under 64 MB in all, .npy headers included
+
+
+def dump_outputs(dirname, outputs, seed=208):
+    """Write `outputs` (name -> device tensor, rows on the first axis) as DIR/<name>.npy: float64 tensors as float64,
+    every other dtype as float32.  When the longest arrays do not fit DUMP_BYTES, all arrays of that length keep the same
+    seeded sample of rows (sorted), so two runs with the same arguments write files that compare row for row."""
+    import torch
+
+    def size(v):
+        return 8 if v.dtype == torch.float64 else 4
+
+    os.makedirs(dirname, exist_ok=True)
+    n = max(v.shape[0] for v in outputs.values())
+    fixed = sum(v.numel() * size(v) for v in outputs.values() if v.shape[0] != n)
+    per_row = sum(v[0].numel() * size(v) for v in outputs.values() if v.shape[0] == n)
+    k = (DUMP_BYTES - fixed) // per_row
+    sample = torch.from_numpy(np.unique(np.random.default_rng(seed).integers(0, n, k))) if n > k else None
+    for name, v in outputs.items():
+        if sample is not None and v.shape[0] == n:
+            v = v.index_select(0, sample.to(v.device))
+        np.save(os.path.join(dirname, f"{name}.npy"), v.cpu().numpy().astype(np.float64 if size(v) == 8 else np.float32))
+
+
 # ---------------------------------------------------------------- C2 / C5: lin_reg, return_pred
 def setup_lin_reg(c):
     from polars_ds_extension_b200 import device as dev
@@ -674,8 +708,12 @@ def setup_lin_reg(c):
                           "thread structure per phase as in the reference (pack / resid / output copies: 1 thread; Gram, X'y, "
                           f"predict: {thr} threads); phases " + ", ".join(f"{k} {s_:.2f}s" for k, s_ in phases.items() if k != "total")}
 
+    def outputs():
+        return {"coeffs": beta[0], "status": status[:1], "pred": pred[0, :rows], "resid": resid[0, :rows]}
+
     path_name = "tcgen05+TMA 3xTF32"
-    return {"step": step, "kernel": kernel, "alg_bytes": rows * (p + 1) * 4, "kernel_name": "moments (Gram X'X | X'y)",
+    return {"step": step, "kernel": kernel, "outputs": outputs, "alg_bytes": rows * (p + 1) * 4,
+            "kernel_name": "moments (Gram X'X | X'y)",
             "traffic": committed_traffic("moments_frame", rows, p), "parity": parity, "e2e": e2e, "cpu": cpu,
             "parallelism": f"row-sharded x{c.world}, one f64 moments all-reduce per step (library NCCL communicator)",
             "config": {"workload": lin_reg_workload(args), "moments_kernel": path_name,
@@ -728,7 +766,8 @@ def setup_c1(c):
         v, dt, sample, cores = cpu_other(args, 50, 3)
         return {"value": v, "unit": "rows/s", "cores": cores, "kind": "port", "sample": sample}
 
-    return {"step": step, "kernel": kernel, "alg_bytes": n * (p + 1) * 8, "kernel_name": "moments f64 (K2a)", "parity": parity,
+    return {"step": step, "kernel": kernel, "outputs": lambda: {"coeffs": beta[0], "status": status[:1]},
+            "alg_bytes": n * (p + 1) * 8, "kernel_name": "moments f64 (K2a)", "parity": parity,
             "e2e": e2e, "cpu": cpu, "l2_policy": "4 MB of input: L2-resident after the first step, latency-bound by design",
             "config": {"workload": f"{args.desc}; step = moments + solve (coefficients)"}}
 
@@ -784,7 +823,8 @@ def setup_grouped(c):
         v, dt, sample, cores = cpu_other(args, 1, 0)
         return {"value": v, "unit": "rows/s", "cores": cores, "kind": "port", "sample": sample}
 
-    return {"step": step, "kernel": step, "alg_bytes": n * (p + 1) * 4, "kernel_name": "grouped moments + batched solve (K5)",
+    return {"step": step, "kernel": step, "outputs": lambda: dict(zip(("coeffs", "status"), state["out"])),
+            "alg_bytes": n * (p + 1) * 4, "kernel_name": "grouped moments + batched solve (K5)",
             "parity": parity, "e2e": e2e, "cpu": cpu, "parallelism": f"groups partitioned over {c.world} ranks, no collective",
             "config": {"workload": f"{args.desc}; {ng} groups of 8000..12000 rows; step = per-group moments + batched solve"}}
 
@@ -838,7 +878,8 @@ def setup_rolling(c):
         v, dt, sample, cores = cpu_other(args, 1, 0)
         return {"value": v, "unit": "rows/s", "cores": cores, "kind": "port", "sample": sample}
 
-    return {"step": step, "kernel": step, "alg_bytes": n * ((p + 1) * 4 + p * 4 + 4 + 1),
+    return {"step": step, "kernel": step, "outputs": lambda: {"coeffs": coeffs, "pred": pred, "valid": valid},
+            "alg_bytes": n * ((p + 1) * 4 + p * 4 + 4 + 1),
             "kernel_name": "rolling window moments + per-row solve (K6, 3 launches)", "parity": parity, "e2e": e2e, "cpu": cpu,
             "parallelism": f"rows partitioned over {c.world} ranks (+ a read-only halo of window-1 rows), no collective",
             "config": {"workload": f"{args.desc}; step = chain sums + scan + per-row window solve, writes coeffs/pred/valid"}}
