@@ -303,6 +303,25 @@ int pdsb_model_fit(int model, const pdsb_matrix* X, const pdsb_matrix* y, int ad
 /* LinearModel::predict (lr/mod.rs:146-174): out[r] = X[r,:] . coeffs[:p] + (has_bias ? coeffs[p] : 0) */
 int pdsb_model_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, double* out);
 
+/* GLM (src/pymodels/py_glm.rs, src/linear/glm/glm_solvers.rs): a family and its canonical link —
+ * gaussian: identity, poisson: log, binomial: logit, gamma: inverse; variances 1, mu, mu (1 - mu), mu^2. */
+enum pdsb_glm_family { PDSB_GLM_GAUSSIAN = 0, PDSB_GLM_POISSON = 1, PDSB_GLM_BINOMIAL = 2, PDSB_GLM_GAMMA = 3 };
+/* GLM::fit by IRLS (faer_irls, glm_solvers.rs:249-359): beta = 0, mu from y, then per iteration the weighted normal
+ * equations X'WX beta = X'Wz by pivoted QR until max|beta - beta_new| < tol or max_iter solves (the last beta is
+ * returned either way).  add_bias appends the ones column last, so the bias is coeffs[n_cols].  At most 64 columns.
+ * coeffs: n_cols + add_bias doubles; *n_iter: the number of weighted least-squares solves. */
+int pdsb_glm_fit(const pdsb_matrix* X, const pdsb_matrix* y, int add_bias, int family, int64_t max_iter, double tol,
+                 double* coeffs, int64_t* n_iter);
+/* GLM predict: g^-1(X coeffs[:p] + bias) (GLM::glm_predict), or the linear predictor itself when linear != 0 */
+int pdsb_glm_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, int family, int linear,
+                     double* out);
+/* Device layer of pdsb_glm_fit: X column-major [n x p] (ldx) and y [n] on the device; X's columns and y must be 16-byte
+ * aligned and ldx even (else an error).  beta: device, p + add_bias doubles.  n_iter: HOST.  Each iteration is one
+ * fused pass over X and y plus a solve on the moments; the call synchronises `stream` once per iteration to test
+ * convergence, and returns when the fit is done. */
+int pdsb_dev_glm_f64(const double* X, int64_t ldx, const double* y, int64_t n, int p, int add_bias, int family,
+                     int64_t max_iter, double tol, double* beta, int64_t* n_iter, void* stream);
+
 /* OnlineLR state ((X'X)^-1 and the coefficients) kept resident on the device between updates. */
 typedef struct pdsb_online_lr pdsb_online_lr;
 pdsb_online_lr* pdsb_online_lr_new(int n_coef, int has_bias);          /* NULL on failure (see pdsb_last_error) */

@@ -33,6 +33,8 @@ class Matrix(C.Structure):
 MODEL_LR, MODEL_ELASTIC_NET, MODEL_ONLINE_LR = range(3)
 METHOD_LSTSQ, METHOD_CD, METHOD_NNLS, METHOD_RCOND, METHOD_INV = range(5)
 SOLVER_QR, SOLVER_SVD, SOLVER_CHOLESKEY = range(3)
+# enum pdsb_glm_family, by the names the reference's GLM class accepts (py_glm.rs / glm_solvers.rs GLMFamily::from)
+GLM_FAMILIES = {"gaussian": 0, "normal": 0, "poisson": 1, "binomial": 2, "logistic": 2, "gamma": 3}
 
 
 def lib() -> C.CDLL:
@@ -77,6 +79,9 @@ def lib() -> C.CDLL:
     mp = C.POINTER(Matrix)
     L.pdsb_model_fit.argtypes = [ci, mp, mp, ci, C.c_char_p, dbl, dbl, dbl, i64, vp, vp]
     L.pdsb_model_predict.argtypes = [mp, vp, ci, ci, vp]
+    L.pdsb_glm_fit.argtypes = [mp, mp, ci, ci, i64, dbl, vp, vp]
+    L.pdsb_glm_predict.argtypes = [mp, vp, ci, ci, ci, ci, vp]
+    L.pdsb_dev_glm_f64.argtypes = [vp, i64, vp, i64, ci, ci, ci, i64, dbl, vp, vp, vp]
     L.pdsb_online_lr_new.restype = vp
     L.pdsb_online_lr_new.argtypes = [ci, ci]
     L.pdsb_online_lr_free.argtypes = [vp]

@@ -36,6 +36,7 @@ SOURCES = [
     "host/multi_gpu.cc",
     "host/lr_host.cc",
     "host/models_host.cc",
+    "host/glm_host.cc",
     "abi/plugin.cc",
 ]
 

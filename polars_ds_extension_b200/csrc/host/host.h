@@ -73,4 +73,9 @@ int world_rank();
 int world_allreduce_f64(double* buf, size_t count, cudaStream_t s);
 int world_allgather_f64(const double* send, double* recv, size_t count, cudaStream_t s);
 
+// GLM by IRLS on a device-resident column-major X and y (glm_host.cc): beta (device, p + add_bias) receives the
+// coefficients, *n_iter the number of weighted least-squares solves.  Synchronises `s` once per iteration.
+int glm_irls(const double* X, int64_t ldx, const double* y, int64_t n, int p, int add_bias, int family, int64_t max_iter,
+             double tol, double* beta, int64_t* n_iter, cudaStream_t s);
+
 }  // namespace pdsb

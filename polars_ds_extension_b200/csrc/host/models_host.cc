@@ -141,7 +141,11 @@ int pdsb_model_fit(int model, const pdsb_matrix* X, const pdsb_matrix* y, int ad
   return 0;
 }
 
-int pdsb_model_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, double* out) {
+}  // extern "C"
+
+namespace {
+// LinearModel::predict (lr/mod.rs:146-174), then g^-1 of `family` (-1: none)
+int predict_matrix(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, int family, double* out) {
   if (require_device()) return 1;
   if (check_matrix(X)) return 1;
   if (n_coef < 1 || !coeffs) { set_error("Matrix is not learned yet."); return 1; }      // lr/mod.rs:149-150
@@ -158,10 +162,52 @@ int pdsb_model_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, i
   PDSB_CUDA_OK(cudaMemcpyAsync(dbeta, coeffs, (size_t)n_coef * sizeof(double), cudaMemcpyHostToDevice, s));
   const double* view = nullptr; int64_t rs = 0, cs = 0;
   if (p > 0 && upload(*X, nullptr, 0, bag, s, &view, &rs, &cs)) return 1;
-  if (predict_strided(view, rs, cs, n, p, dbeta, has_bias ? 1 : 0, dout, s)) return 1;
+  if (predict_strided(view, rs, cs, n, p, dbeta, has_bias ? 1 : 0, family, dout, s)) return 1;
   PDSB_CUDA_OK(cudaMemcpyAsync(out, dout, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, s));
   PDSB_CUDA_OK(cudaStreamSynchronize(s));
   return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int pdsb_model_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, double* out) {
+  return predict_matrix(X, coeffs, n_coef, has_bias, -1, out);
+}
+
+/* GLM::fit (glm_solvers.rs:213-237 -> faer_irls) on numpy matrices: upload to the padded column-major frame, IRLS on
+ * the device (glm_host.cc) */
+int pdsb_glm_fit(const pdsb_matrix* X, const pdsb_matrix* y, int add_bias, int family, int64_t max_iter, double tol,
+                 double* coeffs, int64_t* n_iter) {
+  if (require_device()) return 1;
+  if (check_matrix(X) || check_matrix(y)) return 1;
+  if (!coeffs || !n_iter) { set_error("pdsb_glm_fit: null output"); return 1; }
+  const int64_t n = X->n_rows;
+  const int p = (int)X->n_cols;
+  if (n != y->n_rows || y->n_cols != 1) { set_error("Dimension mismatch."); return 1; }   // lr/mod.rs:122-123
+  if (n == 0 || p == 0 || n < p) { set_error("Not enough rows / columns."); return 1; }   // :124-126
+  if (p > 64) { set_error("glm: more than 64 features are not supported"); return 1; }
+  cudaStream_t s, s2;
+  if (thread_streams(&s, &s2)) return 1;
+  Bag bag(s);
+  const int q = p + (add_bias ? 1 : 0);
+  const int64_t ld = pad_ld(n);
+  double* dZ = bag.alloc((size_t)ld * (p + 1));
+  double* dbeta = bag.alloc((size_t)q);
+  if (!dZ || !dbeta) return 1;
+  const double* v; int64_t a, b;
+  if (upload(*X, dZ, ld, bag, s, &v, &a, &b)) return 1;
+  if (upload(*y, dZ + (size_t)ld * p, ld, bag, s, &v, &a, &b)) return 1;
+  if (glm_irls(dZ, ld, dZ + (size_t)ld * p, n, p, add_bias ? 1 : 0, family, max_iter, tol, dbeta, n_iter, s)) return 1;
+  PDSB_CUDA_OK(cudaMemcpyAsync(coeffs, dbeta, (size_t)q * sizeof(double), cudaMemcpyDeviceToHost, s));
+  PDSB_CUDA_OK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+int pdsb_glm_predict(const pdsb_matrix* X, const double* coeffs, int n_coef, int has_bias, int family, int linear,
+                     double* out) {
+  if (family < PDSB_GLM_GAUSSIAN || family > PDSB_GLM_GAMMA) { set_error("glm: unknown family %d", family); return 1; }
+  return predict_matrix(X, coeffs, n_coef, has_bias, linear ? -1 : family, out);
 }
 
 pdsb_online_lr* pdsb_online_lr_new(int n_coef, int has_bias) {

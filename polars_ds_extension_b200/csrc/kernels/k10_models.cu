@@ -3,11 +3,13 @@
 // (numpy_faer.rs:10-66) to LR::fit / ElasticNet::fit / OnlineLR::{fit, update} and LinearModel::predict
 // (src/linear/lr/mod.rs:146-174).  Fit reuses K2a (moments) + K3 (solve); what is specific to this caller:
 //   gather_colmajor   numpy row-major [n][p] -> the column-major frame the moment kernels read (tiled transpose)
-//   predict_strided   pred = X beta + bias straight from the strided matrix (one pass, no transpose)
+//   predict_strided   pred = X beta + bias straight from the strided matrix (one pass, no transpose); for a GLM the
+//                     inverse link of it (GLM::glm_predict, src/linear/glm/glm_solvers.rs)
 //   woodbury_update   one rank-1 update / downdate of the device-resident (X'X)^-1 and beta
 //                     (woodbury_step, src/linear/online_lr/lr_online_solvers.rs:307-332; OnlineLR::update :85-89)
 #include "../common.h"
 #include "kernels.h"
+#include "glm_link.h"
 
 namespace pdsb {
 
@@ -41,7 +43,7 @@ gather_colmajor_kernel(const T* __restrict__ src, int64_t rs, int64_t cs, int64_
 // one thread per row; beta (<= 256 coefficients) in shared memory
 __global__ void __launch_bounds__(256)
 predict_strided_kernel(const double* __restrict__ X, int64_t rs, int64_t cs, int64_t n, int p,
-                       const double* __restrict__ beta, int has_bias, double* __restrict__ out) {
+                       const double* __restrict__ beta, int has_bias, int family, double* __restrict__ out) {
   extern __shared__ double sb[];
   for (int i = threadIdx.x; i < p + has_bias; i += blockDim.x) sb[i] = beta[i];
   __syncthreads();
@@ -50,7 +52,7 @@ predict_strided_kernel(const double* __restrict__ X, int64_t rs, int64_t cs, int
     const double* row = X + r * rs;
     double acc = bias;
     for (int c = 0; c < p; ++c) acc = fma(row[(int64_t)c * cs], sb[c], acc);
-    out[r] = acc;
+    out[r] = glm::inv_rt(family, acc);
   }
 }
 
@@ -112,10 +114,10 @@ template int gather_colmajor<float>(const float*, int64_t, int64_t, int64_t, int
 template int gather_colmajor<double>(const double*, int64_t, int64_t, int64_t, int, double*, int64_t, cudaStream_t);
 
 int predict_strided(const double* X, int64_t rs, int64_t cs, int64_t n, int p, const double* beta, int has_bias,
-                    double* out, cudaStream_t s) {
+                    int family, double* out, cudaStream_t s) {
   if (n <= 0) return 0;
   const int64_t blocks = std::min<int64_t>(ceil_div(n, 256), (int64_t)sm_count() * 8);
-  predict_strided_kernel<<<(unsigned)blocks, 256, (size_t)(p + 1) * sizeof(double), s>>>(X, rs, cs, n, p, beta, has_bias, out);
+  predict_strided_kernel<<<(unsigned)blocks, 256, (size_t)(p + 1) * sizeof(double), s>>>(X, rs, cs, n, p, beta, has_bias, family, out);
   PDSB_LAUNCH_OK();
   count_launch();
   return 0;

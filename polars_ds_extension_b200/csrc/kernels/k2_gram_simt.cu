@@ -22,6 +22,7 @@
 // Per-(CTA, slice) partials are reduced in a fixed order by a second kernel -> bit-reproducible results.
 #include "../common.h"
 #include "kernels.h"
+#include "glm_link.h"
 
 namespace pdsb {
 
@@ -405,11 +406,27 @@ gram_dmma_wide_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict_
 // the same 16 bytes).  p = 32 needs 10 block pairs instead of the 15 that [X | y | 1] = 34 -> 40 columns cost, p = 8 one
 // instead of 3: the DMMA pipe (37 TFLOP/s measured) is the bound of this path, so the padding columns were the waste.
 // AUX = weights and / or mask present (a missing one is loaded as ones).
-template <typename T, int NB, int DEPTH, int MINB, bool AUX>
+// Rows = where the (y, weight) pair of a row comes from: LoadedRows reads both from memory; GlmRows<F> makes them one
+// IRLS iteration of family F (K2a-GLM): y is the response, and per batch every lane forms its partial eta = x . beta
+// over the feature blocks it holds (beta in NB registers), the 8 column lanes of a row pair add theirs up
+// (shfl_xor 4 / 8 / 16), and the even column lanes evaluate the link for row .x, the odd ones for row .y; the weight
+// w = 1 / (g'(mu)^2 V(mu)) and the working response z = eta + g'(mu) (y - mu) then take the places of (weight, y), so the
+// kernel writes [X | z | 1]' diag(w) [X | z | 1] from ONE read of X and y.
+struct LoadedRows { static constexpr bool kGlm = false; };
+template <int F> struct GlmRows {
+  static constexpr bool kGlm = true;
+  static constexpr int family = F;
+  const double* beta;   // p coefficients (+ the bias last when add_bias) of the current iterate; not read when `first`
+  int add_bias;
+  int first;            // first iteration: eta = g(mu_start(y)) instead of x . beta
+  double mean_y;
+};
+template <typename T, int NB, int DEPTH, int MINB, bool AUX, typename Rows = LoadedRows>
 __global__ void __launch_bounds__(128, MINB)
 gram_dmma_side_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict__ y,
                       const T* __restrict__ w, const T* __restrict__ mask, int64_t n, int p,
-                      double* __restrict__ partials /* [grid][(p+2)^2] */) {
+                      double* __restrict__ partials /* [grid][(p+2)^2] */, Rows src) {
+  constexpr bool WGT = AUX || Rows::kGlm;                 // products carry a per-row weight
   using V = typename Rows2<T>::V;
   constexpr int NP = NB * (NB + 1) / 2;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -433,6 +450,12 @@ gram_dmma_side_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict_
   double xy[NB], x1[NB], yy = 0.0, y1 = 0.0, c11 = 0.0;
 #pragma unroll
   for (int b = 0; b < NB; ++b) { xy[b] = 0.0; x1[b] = 0.0; }
+  double bet[NB], bias = 0.0;
+  if constexpr (Rows::kGlm) {
+#pragma unroll
+    for (int b = 0; b < NB; ++b) bet[b] = (!src.first && live[b]) ? src.beta[8 * b + g] : 0.0;
+    if (!src.first && src.add_bias) bias = src.beta[p];
+  }
 
   struct Batch { V z[NB]; V y, w, m; };
   Batch ring[DEPTH];
@@ -468,11 +491,38 @@ gram_dmma_side_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict_
     double2 z[NB];
 #pragma unroll
     for (int b = 0; b < NB; ++b) z[b] = rows2_f64(q.z[b]);
-    const double2 yv = rows2_f64(q.y), mv = rows2_f64(q.m);
+    double2 yv = rows2_f64(q.y);
+    const double2 mv = rows2_f64(q.m);
     double2 wv = make_double2(1.0, 1.0);
     if constexpr (AUX) wv = rows2_f64(q.w);
+    if constexpr (Rows::kGlm) {
+      constexpr int F = Rows::family;
+      const bool odd = g & 1;                              // this lane evaluates row .y (odd g) or row .x (even g)
+      const double yr = odd ? yv.y : yv.x;
+      double eta, mu;
+      if (src.first) {
+        mu = glm::mu_start<F>(yr, src.mean_y);
+        eta = glm::link<F>(mu);
+      } else {
+        double ex = 0.0, ey = 0.0;
+#pragma unroll
+        for (int b = 0; b < NB; ++b) { ex = fma(z[b].x, bet[b], ex); ey = fma(z[b].y, bet[b], ey); }
+        // xor 4 pairs even and odd g: each keeps the sum of the row it evaluates, then the 4 lanes of its parity add up
+        double e = (odd ? ey : ex) + __shfl_xor_sync(0xffffffffu, odd ? ex : ey, 4);
+        e += __shfl_xor_sync(0xffffffffu, e, 8);
+        e += __shfl_xor_sync(0xffffffffu, e, 16);
+        eta = e + bias;
+        mu = glm::inv<F>(eta);
+      }
+      double wr, zr;
+      glm::irls_row<F>(eta, mu, yr, wr, zr);
+      if (mv.x == 0.0) { wr = 0.0; zr = 0.0; }             // rows past n (a batch is all in or all out)
+      const double wo = __shfl_xor_sync(0xffffffffu, wr, 4), zo = __shfl_xor_sync(0xffffffffu, zr, 4);
+      wv = odd ? make_double2(wo, wr) : make_double2(wr, wo);
+      yv = odd ? make_double2(zo, zr) : make_double2(zr, zo);
+    }
     double2 wy, wm;                                        // w y, w m (the weight enters every product once)
-    if constexpr (AUX) { wy = make_double2(wv.x * yv.x, wv.y * yv.y); wm = make_double2(wv.x * mv.x, wv.y * mv.y); }
+    if constexpr (WGT) { wy = make_double2(wv.x * yv.x, wv.y * yv.y); wm = make_double2(wv.x * mv.x, wv.y * mv.y); }
     else { wy = yv; wm = mv; }
     yy = fma(wy.x, yv.x, fma(wy.y, yv.y, yy));
     y1 = fma(wy.x, mv.x, fma(wy.y, mv.y, y1));
@@ -483,7 +533,7 @@ gram_dmma_side_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict_
     for (int i = 0; i < NB; ++i) {
       xy[i] = fma(z[i].x, wy.x, xy[i]);
       x1[i] = fma(z[i].x, wm.x, x1[i]);
-      const double a0 = AUX ? z[i].x * wv.x : z[i].x;
+      const double a0 = WGT ? z[i].x * wv.x : z[i].x;
 #pragma unroll
       for (int j = i; j < NB; ++j) { dmma884(acc[idx][0], acc[idx][1], a0, z[j].x); ++idx; }
     }
@@ -492,7 +542,7 @@ gram_dmma_side_kernel(const T* __restrict__ X, int64_t ldx, const T* __restrict_
     for (int i = 0; i < NB; ++i) {
       xy[i] = fma(z[i].y, wy.y, xy[i]);
       x1[i] = fma(z[i].y, wm.y, x1[i]);
-      const double a1 = AUX ? z[i].y * wv.y : z[i].y;
+      const double a1 = WGT ? z[i].y * wv.y : z[i].y;
 #pragma unroll
       for (int j = i; j < NB; ++j) { dmma884(acc[idx][0], acc[idx][1], a1, z[j].y); ++idx; }
     }
@@ -585,7 +635,8 @@ constexpr int wide_depth(int nb, bool aux) {
   return aux ? auxd[nb - 1] : plain[nb - 1];
 }
 
-template <typename T> using SideFn = void (*)(const T*, int64_t, const T*, const T*, const T*, int64_t, int, double*);
+template <typename T, typename R = LoadedRows>
+using SideFn = void (*)(const T*, int64_t, const T*, const T*, const T*, int64_t, int, double*, R);
 template <typename T> using WideFn = void (*)(const T*, int64_t, const T*, int64_t, const T*, const T*, int64_t, int, int, double*);
 
 #ifdef PDSB_K2A_SWEEP   // sweep build (profiles/_ab): every depth 2..9 is instantiated, PDSB_K2A_DEPTH picks one per call
@@ -711,7 +762,7 @@ static int moments_dmma(const T* X, int64_t ldx, const T* Y, int64_t ldy, const 
   if (dev_alloc((void**)&partials, (size_t)(grid_main + grid_tail) * q1 * q1 * sizeof(double), s)) return 1;
   int rc = 0;
   if (side) {
-    sfn<<<grid_main, 128, ring_smem, s>>>(X, ldx, Y, w, mask, n_main, p, partials);
+    sfn<<<grid_main, 128, ring_smem, s>>>(X, ldx, Y, w, mask, n_main, p, partials, LoadedRows{});
     cudaError_t e = cudaGetLastError();
     count_launch();
     if (e != cudaSuccess) { set_error("gram_dmma_side launch failed: %s", cudaGetErrorString(e)); rc = 1; }
@@ -816,6 +867,110 @@ int moments_simt(const T* X, int64_t ldx, const T* Y, int64_t ldy, const T* w, c
   dev_free(partials, s);
   if (e != cudaSuccess) { set_error("reduce_partials launch failed: %s", cudaGetErrorString(e)); return 1; }
   return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// K2a-GLM: the moments of one IRLS iteration, [X | z | 1]' diag(w) [X | z | 1] with (w, z) computed from (X, y, beta)
+// on the fly — the side kernel with GlmRows<F> for the rows n - n % 8, glm_rows_kernel for the rest.  X: column-major,
+// 16-byte aligned columns, even ldx; y 16-byte aligned (the caller checks).
+//
+// Ring depth per NB: the plain side kernel's depth where that compiles without a spill, shallower where beta's NB
+// registers would push it into one (ptxas -v, sm_100a).
+constexpr int glm_depth(int nb) {
+  constexpr int d[8] = {2, 8, 6, 3, 2, 2, 2, 2};
+  return d[nb - 1];
+}
+template <int F, int NB> static SideFn<double, GlmRows<F>> glm_fn() {
+  return gram_dmma_side_kernel<double, NB, glm_depth(NB), 2, false, GlmRows<F>>;
+}
+template <int F> static SideFn<double, GlmRows<F>> glm_fn_rt(int nb) {
+  switch (nb) {
+    case 1: return glm_fn<F, 1>(); case 2: return glm_fn<F, 2>(); case 3: return glm_fn<F, 3>(); case 4: return glm_fn<F, 4>();
+    case 5: return glm_fn<F, 5>(); case 6: return glm_fn<F, 6>(); case 7: return glm_fn<F, 7>(); default: return glm_fn<F, 8>();
+  }
+}
+
+// The last n % 8 (< 8) rows: one CTA; (w, z) of each row first, then one thread per entry of the partial, in
+// gram_rows_kernel's order.
+template <int F>
+__global__ void __launch_bounds__(128)
+glm_rows_kernel(const double* __restrict__ X, int64_t ldx, const double* __restrict__ y, int rows, int p, GlmRows<F> src,
+                double* __restrict__ out /* [(p+2)^2] */) {
+  __shared__ double sw[8], sz[8];
+  const int q1 = p + 2;
+  if ((int)threadIdx.x < rows) {
+    const int r = threadIdx.x;
+    double eta, mu;
+    if (src.first) {
+      mu = glm::mu_start<F>(y[r], src.mean_y);
+      eta = glm::link<F>(mu);
+    } else {
+      eta = 0.0;
+      for (int c = 0; c < p; ++c) eta = fma(X[(int64_t)c * ldx + r], src.beta[c], eta);
+      if (src.add_bias) eta += src.beta[p];
+      mu = glm::inv<F>(eta);
+    }
+    glm::irls_row<F>(eta, mu, y[r], sw[r], sz[r]);
+  }
+  __syncthreads();
+  auto at = [&](int c, int r) -> double { return c < p ? X[(int64_t)c * ldx + r] : (c == p ? sz[r] : 1.0); };
+  for (int e = threadIdx.x; e < q1 * q1; e += blockDim.x) {
+    const int a = e / q1, b = e % q1;
+    double v = 0.0;
+    for (int r = 0; r < rows; ++r) v = fma(sw[r], at(a, r) * at(b, r), v);
+    out[e] = v;
+  }
+}
+
+template <int F>
+static int glm_moments_t(const double* X, int64_t ldx, const double* y, int64_t n, int p, int add_bias, const double* beta,
+                         int first, double mean_y, double* M, cudaStream_t s) {
+  const int q1 = p + 2;
+  const GlmRows<F> src{beta, add_bias, first, mean_y};
+  const int64_t n_main = n - n % 8, n_tail = n - n_main;
+  SideFn<double, GlmRows<F>> fn = glm_fn_rt<F>((p + 7) / 8);
+  const size_t ring_smem = ring_kernel_smem((p + 7) / 8);
+  int per_sm = 2;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, 128, ring_smem) != cudaSuccess || per_sm < 1) {
+    (void)cudaGetLastError();
+    per_sm = 2;
+  }
+  const int grid_main = n_main ? (int)std::min<int64_t>(ceil_div(n_main, 32), (int64_t)sm_count() * per_sm) : 0;
+  const int nparts = grid_main + (n_tail > 0 ? 1 : 0);
+  double* partials = nullptr;
+  if (dev_alloc((void**)&partials, (size_t)nparts * q1 * q1 * sizeof(double), s)) return 1;
+  cudaError_t e = cudaSuccess;
+  if (grid_main) {
+    fn<<<grid_main, 128, ring_smem, s>>>(X, ldx, y, nullptr, nullptr, n_main, p, partials, src);
+    e = cudaGetLastError();
+    count_launch();
+  }
+  if (e == cudaSuccess && n_tail) {
+    glm_rows_kernel<F><<<1, 128, 0, s>>>(X + n_main, ldx, y + n_main, (int)n_tail, p, src,
+                                         partials + (size_t)grid_main * q1 * q1);
+    e = cudaGetLastError();
+    count_launch();
+  }
+  if (e == cudaSuccess) {
+    reduce_partials_kernel<<<q1 * q1, 128, 0, s>>>(partials, nparts, q1 * q1, M);
+    e = cudaGetLastError();
+    count_launch();
+  }
+  dev_free(partials, s);
+  if (e != cudaSuccess) { set_error("glm moments launch failed: %s", cudaGetErrorString(e)); return 1; }
+  return 0;
+}
+
+int glm_moments(const double* X, int64_t ldx, const double* y, int64_t n, int p, int add_bias, int family,
+                const double* beta, int first, double mean_y, double* M, cudaStream_t s) {
+  if (p < 1 || p > 64) { set_error("glm: %d features are not supported (1..64)", p); return 1; }
+  switch (family) {
+    case glm::GAUSSIAN: return glm_moments_t<glm::GAUSSIAN>(X, ldx, y, n, p, add_bias, beta, first, mean_y, M, s);
+    case glm::POISSON: return glm_moments_t<glm::POISSON>(X, ldx, y, n, p, add_bias, beta, first, mean_y, M, s);
+    case glm::BINOMIAL: return glm_moments_t<glm::BINOMIAL>(X, ldx, y, n, p, add_bias, beta, first, mean_y, M, s);
+    case glm::GAMMA: return glm_moments_t<glm::GAMMA>(X, ldx, y, n, p, add_bias, beta, first, mean_y, M, s);
+    default: set_error("glm: unknown family %d", family); return 1;
+  }
 }
 
 template int moments_simt<float>(const float*, int64_t, const float*, int64_t, const float*, const float*,

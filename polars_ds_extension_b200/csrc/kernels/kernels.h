@@ -11,6 +11,12 @@ template <typename T>
 int moments_simt(const T* X, int64_t ldx, const T* Y, int64_t ldy, const T* w, const T* mask, int64_t n,
                  int p, int t, double* M, cudaStream_t s, int64_t bstride = 0 /* frame block stride (elements) or 0 */);
 
+// K2a-GLM: moments [X | z | 1]' diag(w) [X | z | 1] of one IRLS iteration of `family` (enum pdsb_glm_family), (w, z)
+// computed in the kernel from X, y and beta (first != 0: from mu_start(y, mean_y), beta not read).  p <= 64; X columns and
+// y 16-byte aligned, ldx even.
+int glm_moments(const double* X, int64_t ldx, const double* y, int64_t n, int p, int add_bias, int family,
+                const double* beta, int first, double mean_y, double* M, cudaStream_t s);
+
 // K2b tcgen05 + TMA moments, f32, 3xTF32 split (hi/lo), f64 flush; p <= 64 features, t <= 4 targets.  Returns 0 ok, 1 error,
 // -1 "shape not supported by this kernel" (caller uses K2a).
 int moments_tcgen05_f32(const float* X, int64_t ldx, const float* Y, int64_t ldy, const float* mask,
@@ -71,8 +77,9 @@ int online_lin_reg(const T* X, int64_t ldx, const T* y, int64_t n, int p, int ad
 // K10 dense-matrix callers (model classes): strided gather to column-major, strided predict, Woodbury update
 template <typename T>
 int gather_colmajor(const T* src, int64_t rs, int64_t cs, int64_t n, int p, T* dst, int64_t ld, cudaStream_t s);
+// family: enum pdsb_glm_family whose inverse link is applied to X beta + bias; -1 (or gaussian) leaves it as is
 int predict_strided(const double* X, int64_t rs, int64_t cs, int64_t n, int p, const double* beta, int has_bias,
-                    double* out, cudaStream_t s);
+                    int family, double* out, cudaStream_t s);
 int woodbury_update(double* inv, double* w, int q, int has_bias, const double* x, double y, double c, cudaStream_t s);
 
 // K11 logistic regression (IRLS row pass: weights, working response, summed log-loss per block; probabilities)

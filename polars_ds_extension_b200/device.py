@@ -11,8 +11,8 @@ from typing import Optional, Tuple
 
 import torch
 
-from ._lib import (METHOD_CD, METHOD_INV, METHOD_LSTSQ, METHOD_NNLS, METHOD_RCOND, SOLVER_CHOLESKEY, SOLVER_QR,
-                   SOLVER_SVD, SolveOpts, check, lib)
+from ._lib import (GLM_FAMILIES, METHOD_CD, METHOD_INV, METHOD_LSTSQ, METHOD_NNLS, METHOD_RCOND, SOLVER_CHOLESKEY,
+                   SOLVER_QR, SOLVER_SVD, SolveOpts, check, lib)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -124,6 +124,23 @@ def recursive_shard(X: torch.Tensor, y: torch.Tensor, min_rows: int, m0: Optiona
     check(fn(_ptr(X), _ld(X), _ptr(y), n, p, int(add_bias), min_rows, int(skip), float(l2_reg),
              _ptr(m0) if m0 is not None else None, row0, _ptr(coeffs), _ptr(pred), _ptr(valid), _stream()))
     return coeffs, pred, valid
+
+
+def glm(X: torch.Tensor, y: torch.Tensor, family: str = "normal", add_bias: bool = False, max_iter: int = 100,
+        tol: float = 1e-8, n: Optional[int] = None) -> Tuple[torch.Tensor, int]:
+    """GLM by IRLS on float64 tensors: X (p, ld), y (1, ld) or (ld,).  Returns (beta, n_iter): beta is a (p + add_bias,)
+    float64 tensor on X's device, bias last; n_iter the number of weighted least-squares solves.  X's rows and y must
+    start 16-byte aligned and ld must be even (torch allocations with an even ld are)."""
+    if family not in GLM_FAMILIES:
+        raise NotImplementedError(f"unknown GLM family {family!r}")
+    p = X.shape[0]
+    n = X.shape[1] if n is None else n
+    yv = y.reshape(1, -1) if y.dim() == 1 else y
+    beta = torch.empty(p + int(add_bias), dtype=torch.float64, device=X.device)
+    it = C.c_int64(0)
+    check(lib().pdsb_dev_glm_f64(_ptr(X), _ld(X), _ptr(yv), n, p, int(add_bias), GLM_FAMILIES[family], int(max_iter),
+                                 float(tol), _ptr(beta), C.byref(it), _stream()))
+    return beta, int(it.value)
 
 
 FRAME_ROWS = 128

@@ -1,4 +1,4 @@
-"""Model classes over the B200 engine: `LR`, `ElasticNet`, `OnlineLR`.
+"""Model classes over the B200 engine: `LR`, `ElasticNet`, `OnlineLR`, `GLM`.
 
 Mirror of the reference's numpy-facing classes (/root/reference/python/polars_ds/linear_models.py:134-700), which are
 thin wrappers over the PyO3 types PyLR / PyElasticNet / PyOnlineLR (src/pymodels/py_lr.rs:21-224).  Same constructor
@@ -6,8 +6,11 @@ arguments, method names, null policies and error messages; the arithmetic runs i
 `pdsb_model_predict`, `pdsb_online_lr_*` in include/pdsb.h): moments + solve on the device, Woodbury updates on
 device-resident state.  There is no CPU path: without the shared library or a CUDA device every fit / predict raises.
 
+`GLM` (linear_models.py:700-950; PyGLM, src/pymodels/py_glm.rs) fits by IRLS on the device (`pdsb_glm_fit`): one fused
+pass over X and y per iteration builds the weighted moments, a pivoted-QR solve on them gives the next iterate.
+
 Data frames: `fit_df` / `predict_df` accept this package's Arrow-backed `Frame` (and a Polars frame when polars is
-installed); GLM and MixedModel of the reference file are outside this engine's scope (SURVEY.md §8f).
+installed); MixedModel of the reference file is outside this engine's scope (SURVEY.md §8f).
 """
 from __future__ import annotations
 
@@ -16,10 +19,10 @@ from typing import Any, List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from ._lib import MODEL_ELASTIC_NET, MODEL_LR, MODEL_ONLINE_LR, Matrix, lib
+from ._lib import GLM_FAMILIES, MODEL_ELASTIC_NET, MODEL_LR, MODEL_ONLINE_LR, Matrix, lib
 from .typing import LRSolverMethods, NullPolicy
 
-__all__ = ["LR", "ElasticNet", "OnlineLR"]
+__all__ = ["LR", "ElasticNet", "OnlineLR", "GLM"]
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -373,3 +376,70 @@ class OnlineLR:
     def predict(self, X: np.ndarray) -> np.ndarray:
         w, _ = self._get()
         return _predict(X, w, self._has_bias)
+
+
+# GLM::to_string (glm_solvers.rs): the Debug names of the family's link and variance functions
+_GLM_NAMES = {0: ("Identity", "Gaussian"), 1: ("Log", "Poisson"), 2: ("Logit", "Binomial"), 3: ("Inverse", "Gamma")}
+
+
+class GLM(_Base):
+    """Generalized linear model with the canonical link of its family, fit by IRLS (linear_models.py:700-950; PyGLM,
+    py_glm.rs): gaussian / normal -> identity, poisson -> log, binomial / logistic -> logit, gamma -> inverse.  With
+    `add_bias` the bias is the last coefficient.  At most 64 features."""
+
+    def __init__(self, add_bias: bool = False, solver: str = "irls", family: str = "normal", max_iter: int = 100,
+                 tol: float = 1e-8, feature_names_in_: Optional[List[str]] = None):
+        if solver not in ["irls"]:
+            raise NotImplementedError
+        if max_iter < 1:
+            raise ValueError("`max_iter` must be > 1.")
+        if family not in ["gaussian", "normal", "poisson", "binomial", "logistic", "gamma"]:
+            raise NotImplementedError
+        self._has_bias = bool(add_bias)
+        self.solver = solver
+        self.family = family
+        self.max_iter = int(max_iter)
+        self.tol = abs(float(tol))
+        self._family = GLM_FAMILIES[family]
+        self._fitted = None
+        self._n_iter = 0          # weighted least-squares solves of the last fit
+        self.feature_names_in_ = [] if feature_names_in_ is None else list(feature_names_in_)
+
+    def __repr__(self) -> str:
+        # The reference calls PyGLM.describe(), which does not exist (AttributeError); this is GLM::to_string's text.
+        link, variance = _GLM_NAMES[self._family]
+        return f"GLM:\nLink: {link}\nVariance: {variance}"
+
+    def _run(self, X: np.ndarray, y: np.ndarray):
+        Xm, ym = _as_matrix(X), _as_matrix(y)
+        coeffs = np.empty(Xm.shape[1] + int(self._has_bias), dtype=np.float64)
+        it = C.c_int64(0)
+        xv, yv = _view(Xm), _view(ym)
+        _call(lib().pdsb_glm_fit(C.byref(xv), C.byref(yv), int(self._has_bias), self._family, self.max_iter, self.tol,
+                                 coeffs.ctypes.data, C.byref(it)))
+        self._fitted, self._n_iter = coeffs, int(it.value)
+        return self
+
+    def fit(self, X: np.ndarray, y: np.ndarray, null_policy: NullPolicy = "ignore"):
+        X_, y_ = _handle_nans_in_np(_as_matrix(X), _as_matrix(y).reshape((-1, 1)), null_policy)
+        return self._run(X_, y_)
+
+    def fit_df(self, df: Any, features: List[str], target: str, null_policy: NullPolicy = "skip",
+               show_report: bool = False):
+        X, y = _df_to_xy(df, list(features), target, null_policy)
+        self.feature_names_in_ = list(features)
+        return self._run(X, y)
+
+    def predict_df(self, df: Any, name: str = "prediction"):
+        raise NotImplementedError("GLM.predict_df is not available (the reference leaves it out too)")
+
+    def predict(self, X: np.ndarray, linear: bool = False) -> np.ndarray:
+        """g^-1(X beta + bias) as an (n, 1) array; the linear predictor X beta + bias itself when `linear`."""
+        if not self.is_fit():
+            raise ValueError("Matrix is not learned yet.")
+        Xm = _as_matrix(X)
+        out = np.empty((Xm.shape[0], 1), dtype=np.float64)
+        xv = _view(Xm)
+        _call(lib().pdsb_glm_predict(C.byref(xv), self._fitted.ctypes.data, int(self._fitted.size), int(self._has_bias),
+                                     self._family, int(bool(linear)), out.ctypes.data))
+        return out
